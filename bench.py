@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the OMG two-stage SDXL denoising hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is ONE IMAGE through the whole hot path as the reference executes it (config 2): stage 1 (30 steps, main
 UNet B=4) + stage 2 (30 steps, main UNet B=4, and for step index > 15 two concept UNets B=2 with un-merged LoRA) =
@@ -17,6 +17,9 @@ UNet B=4) + stage 2 (30 steps, main UNet B=4, and for step index > 15 two concep
   sample-forward at the same latent size, extrapolated to images/sec (= 1 / (296 * t)).
 N > 1: independent images, one replica per GPU (weights broadcast once over NCCL, final latents all-gathered);
 scaling is weak (K images per GPU).
+--dump-outputs DIR: after the timed steps, rank 0 writes the latents its last timed image returned as float32
+DIR/stage1_latents.npy and DIR/stage2_latents.npy (2 x 4 x 128 x 128 each).  Weights, prompts, masks and the noise of
+every image are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -204,7 +207,13 @@ def _main():
     ap.add_argument("--total-images", type=int, default=0,
                     help="BASELINE config 5: this many independent images (seeds 0..N-1) sharded image j -> rank j mod G "
                          "(strong scaling); overrides --steps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latents of the last timed image to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -322,6 +331,11 @@ def _main():
         dist.all_reduce(lt, op=dist.ReduceOp.SUM)
         launches = int(lt.item())
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in zip(("stage1_latents", "stage2_latents"), outs[-1]):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
     ms_e2e, outs_h = (float("nan"), None) if args.skip_e2e else timed(args.steps, host, True)
     if world > 1:  # gather final latents (128 KiB per image) on every rank
         mine = torch.stack([o[1] for o in outs]).to(dev)
