@@ -39,6 +39,10 @@ typedef struct {
 
 enum { OMG_EPI_NONE = 0, OMG_EPI_GEGLU = 1, OMG_EPI_SILU = 2, OMG_EPI_QUICK_GELU = 3, OMG_EPI_GELU = 4, OMG_EPI_GELU_TANH = 5 };
 
+/* Element type of the 16-bit operands of omg_gemm (omg_gemm_desc.dtype).  bf16 has fp32's exponent range: the VAE decoder
+ * runs it for weights whose activations overflow fp16 (the original SDXL VAE, which diffusers up-casts to fp32). */
+enum { OMG_DTYPE_F16 = 0, OMG_DTYPE_BF16 = 1 };
+
 /*
  * out[pix, n] = epi( sum_seg sum_k A_seg[pix+(dx,dy), k] * W[n, b_k0+k] + bias[n] + rowvec[b, n] ) + residual[pix, n]
  *
@@ -105,6 +109,11 @@ typedef struct {
     int64_t residual_f32_ld;
     void* out_f32;
     int64_t out_f32_ld;
+    /* OMG_DTYPE_F16 (0, what a zeroed descriptor has) or OMG_DTYPE_BF16: the type of every 16-bit operand of the call -
+     * A views, w, w2, bias, residual and the output.  bf16 supports OMG_EPI_NONE with bias, residual, K-segments, shifted
+     * and strided views and every tile shape; activations / GEGLU, folded LayerNorm (row_stats_*), col_stats_out, rowvec,
+     * weight planes / column groups and the fp32 twins are rejected. */
+    int32_t dtype;
 } omg_gemm_desc;
 
 int omg_gemm(const omg_gemm_desc* desc, void* stream);
@@ -156,6 +165,9 @@ int omg_attention(const omg_attn_desc* desc, void* stream);
 #define OMG_GN_WS_FLOATS(B) ((B) * (2 * 2 * 2560 + 64 * OMG_GN_MAX_SPLITS))
 int omg_groupnorm(const void* x1, int C1, const void* x2, int C2, int B, int HW, const void* gamma, const void* beta,
                   float eps, int silu, void* stats_ws, void* y, void* stream);
+/* omg_groupnorm with bf16 x1, x2, gamma, beta and y (same contract, fp32 statistics). */
+int omg_groupnorm_bf16(const void* x1, int C1, const void* x2, int C2, int B, int HW, const void* gamma, const void* beta,
+                       float eps, int silu, void* stats_ws, void* y, void* stream);
 
 /* Per-channel (sum, sum of squares) partials of a stored channels-last tensor x [B, HW, C], one float2 per channel per
  * 32-row block: out [B][ceil(HW/32)][C] - the layout omg_gemm's col_stats_out produces (for tensors that were modified
@@ -218,6 +230,8 @@ int omg_axpy(const void* a, const void* b, float alpha, void* y, long long n, vo
  * 512 channels: `Attention(heads=1)` inside diffusers' AutoencoderKL, reached from src/pipelines/lora_pipeline.py:649)
  * materialises its scores with omg_gemm, normalises them here and applies them with a second omg_gemm. */
 int omg_softmax_rows(void* x, long long rows, int cols, long long ld, float scale, void* stream);
+/* omg_softmax_rows over a bf16 matrix (same contract). */
+int omg_softmax_rows_bf16(void* x, long long rows, int cols, long long ld, float scale, void* stream);
 
 /*
  * EfficientViT-SAM image encoder (the segmentation model between the two stages; SURVEY 8f-4), the ops that are not

@@ -2,7 +2,7 @@
 """OMG + InstantID multi-identity generation on the B200 path.  The reference CLI's flags (names, defaults, types:
 inference_instantid.py:259-286, pinned by tests/golden/cli_flags.json), prompt mini-DSL, two-stage flow and output
 files; additions (non-breaking): --synthetic, --tiny, --num_inference_steps, --image_size, --dedup, --mask_boxes,
---face_embeds, --face_kps.
+--face_embeds, --face_kps, --vae.
 
 Face analysis (insightface antelopev2), segmentation and the VAE sit outside the accelerated hot path (SURVEY section
 8): when `insightface` is not importable the identities come from --face_embeds (one 512-d .pt / .npy per region) and
@@ -98,6 +98,9 @@ def parse_args():
                    "(replaces insightface on the reference images)")
     p.add_argument("--face_kps", default="", type=str, help="JSON file: list of five (x, y) key-points per face for "
                    "the stage-2 IdentityNet condition (replaces insightface on the stage-1 image)")
+    p.add_argument("--vae", default="", type=str, help="diffusers VAE directory, or a checkpoint root with vae/: decode "
+                   "both stages to PNG on the GPU, in bf16 when its config.json has force_upcast (the original SDXL VAE), "
+                   "else fp16 (without it the latents are saved)")
     return p.parse_args()
 
 
@@ -243,6 +246,10 @@ if __name__ == "__main__":
             masks.append(m)
         masks = masks or [None] * len(regions)
     pipe.dedup = args.dedup
+    if args.vae:
+        from omg_b200.vae import PackedVaeDecoder
+        pipe.vae_decoder = PackedVaeDecoder.from_pretrained(args.vae, device=device)
+        kwargs["output_type"] = "pil"  # VAE decode + postprocess
     input_prompt = [prompts, regions]
     common = dict(input_prompt=input_prompt, concept_models=cm, input_neg_prompt=[args.negative_prompt] * len(input_prompt),
                   controller=controller, face_app=face_app, controlnet_conditioning_scale=args.IdentityNet_rate,
@@ -264,6 +271,9 @@ if __name__ == "__main__":
     os.makedirs(save_dir, exist_ok=True)
     print(f"save to: {save_dir}")
     for idx, name in ((0, "stage-1"), (1, "stage-2")):
-        torch.save(image[idx].cpu(), os.path.join(save_dir, name + ".pt"))
+        if args.vae:
+            image[idx].save(os.path.join(save_dir, name + ".png"))
+        else:
+            torch.save(image[idx].cpu(), os.path.join(save_dir, name + ".pt"))
     with open(os.path.join(save_dir, f"**---{args.suffix}---{hash_code}.txt"), "w") as fw:
         fw.writelines(configs)

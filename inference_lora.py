@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """OMG + LoRA multi-concept generation on the B200 path.  Same flags, prompt mini-DSL, two-stage flow and output
 files as the reference CLI (inference_lora.py:201-323); additions (non-breaking): --synthetic, --num_inference_steps,
---image_size, --mask_boxes, --vae_fp16_safe.
+--image_size, --mask_boxes, --vae_fp16_safe, --vae.
 
 The segmentation models between the stages (YOLO-World / GroundingDINO + SAM) and the VAE / text encoders are outside
 the accelerated hot path (SURVEY section 8): masks come from --mask_boxes (x0,y0,x1,y1 per concept, '|' separated) or,
@@ -72,8 +72,12 @@ def parse_args():
     p.add_argument("--tiny", action="store_true", help="with --synthetic: toy widths (plumbing check)")
     p.add_argument("--decode", action="store_true", help="with --synthetic: decode with a random-init VAE decoder")
     p.add_argument("--mask_boxes", default="", type=str, help="x0,y0,x1,y1|x0,y0,x1,y1 (pixels), replaces segmentation")
-    p.add_argument("--vae_fp16_safe", default="", type=str, help="directory of fp16-safe SDXL VAE weights: decode to "
-                   "PNG on the GPU (without it the latents are saved)")
+    vae = p.add_mutually_exclusive_group()
+    vae.add_argument("--vae_fp16_safe", default="", type=str, help="directory of fp16-safe SDXL VAE weights: decode to "
+                     "PNG on the GPU (without it the latents are saved)")
+    vae.add_argument("--vae", default="", type=str, help="diffusers VAE directory, or a checkpoint root with vae/: decode "
+                     "both stages to PNG on the GPU, in bf16 when its config.json has force_upcast (the original SDXL VAE), "
+                     "else fp16")
     return p.parse_args()
 
 
@@ -165,6 +169,9 @@ if __name__ == "__main__":
         from omg_b200.vae import PackedVaeDecoder, VaeConfig
         vcfg = VaeConfig.tiny() if args.tiny else VaeConfig.sdxl()
         pipe.vae_decoder = PackedVaeDecoder(synthetic.make_vae_state_dict(vcfg, 0), vcfg, device=device)
+    if args.vae:
+        from omg_b200.vae import PackedVaeDecoder
+        pipe.vae_decoder = PackedVaeDecoder.from_pretrained(args.vae, device=device)
     decoded = pipe.vae_decoder is not None
     if decoded:
         kwargs["output_type"] = "pil"  # lora_pipeline.py:634-661: VAE decode + postprocess

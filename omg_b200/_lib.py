@@ -11,6 +11,7 @@ OMG_MAX_SEGS = 12
 OMG_ATTN_MAX_ITEMS = 16
 OMG_MAX_CONCEPTS = 8
 EPI_NONE, EPI_GEGLU, EPI_SILU, EPI_QUICK_GELU, EPI_GELU, EPI_GELU_TANH = 0, 1, 2, 3, 4, 5
+DTYPE_F16, DTYPE_BF16 = 0, 1
 
 
 class View4(C.Structure):
@@ -33,7 +34,8 @@ class GemmDesc(C.Structure):
                 ("row_stats_stride", C.c_int64), ("ln_dim", C.c_int32), ("ln_eps", C.c_float), ("col_c1", C.c_void_p), ("col_c2", C.c_void_p),
                 ("n_col_groups", C.c_int32), ("col_group_end", C.c_int64 * 8), ("w_group_planes", C.c_int32), ("cta_pair", C.c_int32),
                 ("col_stats_out", C.c_void_p), ("col_stats_rb0", C.c_int32), ("col_stats_rb_total", C.c_int32),
-                ("residual_f32", C.c_void_p), ("residual_f32_ld", C.c_int64), ("out_f32", C.c_void_p), ("out_f32_ld", C.c_int64)]
+                ("residual_f32", C.c_void_p), ("residual_f32_ld", C.c_int64), ("out_f32", C.c_void_p), ("out_f32_ld", C.c_int64),
+                ("dtype", C.c_int32)]
 
 
 class AttnDesc(C.Structure):
@@ -68,12 +70,15 @@ SYMBOLS = {
     "omg_attention": (C.c_int, [C.POINTER(AttnDesc), C.c_void_p]),
     "omg_groupnorm": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "omg_groupnorm_bf16": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                     C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "omg_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_float,
                                 C.c_void_p]),
     "omg_fuse_step": (C.c_int, [C.POINTER(FuseDesc), C.c_void_p]),
     "omg_ctx_mix": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "omg_axpy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_longlong, C.c_void_p]),
     "omg_softmax_rows": (C.c_int, [C.c_void_p, C.c_longlong, C.c_int, C.c_longlong, C.c_float, C.c_void_p]),
+    "omg_softmax_rows_bf16": (C.c_int, [C.c_void_p, C.c_longlong, C.c_int, C.c_longlong, C.c_float, C.c_void_p]),
     "omg_dwconv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                              C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "omg_group1x1": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),

@@ -917,13 +917,13 @@ static int launch_cross(AttnParams& p, const omg_attn_desc* d, cudaStream_t stre
         const uint64_t dims[3] = {(uint64_t)(d->k_col0 + cols), (uint64_t)d->n_kv, (uint64_t)(max_kb + 1)};
         const uint64_t strides[3] = {1, (uint64_t)d->k_ld, (uint64_t)d->k_bs};
         const uint32_t box[3] = {64, NK, 1};
-        if (make_tmap_f16(&p.k_map, d->k, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (make_tmap_16b(&p.k_map, d->k, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
     }
     {
         const uint64_t dims[3] = {(uint64_t)(d->v_col0 + cols), (uint64_t)d->n_kv, (uint64_t)(max_vb + 1)};
         const uint64_t strides[3] = {1, (uint64_t)d->v_ld, (uint64_t)d->v_bs};
         const uint32_t box[3] = {64, NK, 1};
-        if (make_tmap_f16(&p.v_map, d->v, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (make_tmap_16b(&p.v_map, d->v, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
     }
     // heads per CTA: as many as keep the grid at >= ~1.5 CTAs per SM slot pair (148 SMs x 2), at most 8
     const int tiles = ((d->n_q + ATT_BQ - 1) / ATT_BQ) * d->n_items;
@@ -948,7 +948,7 @@ static int make_attn_map(CUtensorMap* m, const void* ptr, int cols, int ld, int 
     const uint64_t dims[3] = {(uint64_t)cols, (uint64_t)tokens, (uint64_t)nb};
     const uint64_t strides[3] = {1, (uint64_t)ld, (uint64_t)bs};
     const uint32_t box[3] = {64, box_rows, 1};
-    return make_tmap_f16(m, ptr, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
+    return make_tmap_16b(m, ptr, 3, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 }  // namespace omg

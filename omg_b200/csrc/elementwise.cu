@@ -5,7 +5,10 @@
 // forcing a host sync through nonzero(); src/pipelines/instantid_pipeline.py:618-690 is identical).
 // Algorithmic bytes per launch (HW latent pixels, n concepts): read (4 + 2n) * HW*8*2 B noise + n * HW*4 B masks
 // + HW*2*4*4 B latents; write HW*2*4*4 B latents + 6 * HW*8*2 B next inputs.
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
+
+#include <type_traits>
 
 #include "../../include/omg_b200.h"
 #include "host_common.h"
@@ -150,12 +153,14 @@ __global__ void axpy_kernel(const uint4* __restrict__ a, const uint4* __restrict
     y[i] = o;
 }
 
-// In-place softmax(scale * x) over the rows of an fp16 matrix, fp32 arithmetic, one CTA per row, the row kept in
+// In-place softmax(scale * x) over the rows of an fp16 | bf16 matrix, fp32 arithmetic, one CTA per row, the row kept in
 // registers (cols <= 256 threads x MAXV vectors x 8).  Used by the VAE decoder's single-head attention (head_dim 512
 // is outside the flash kernel's d = 64), whose scores are materialised by omg_gemm.
 constexpr int SM_THREADS = 256;
 constexpr int SM_MAXV = 16;  // cols <= 32768
-__global__ void __launch_bounds__(SM_THREADS) softmax_rows_kernel(__half* __restrict__ x, int cols, long long ld, float scale_log2) {
+template <typename T>
+__global__ void __launch_bounds__(SM_THREADS) softmax_rows_kernel(T* __restrict__ x, int cols, long long ld, float scale_log2) {
+    using T2 = typename Pair<T>::type;
     griddep_launch_dependents();
     griddep_wait();
     __shared__ float red[SM_THREADS / 32];
@@ -168,10 +173,10 @@ __global__ void __launch_bounds__(SM_THREADS) softmax_rows_kernel(__half* __rest
         const int j = threadIdx.x + i * SM_THREADS;
         if (j < nvec) {
             v[i] = row[j];
-            const __half2* h = reinterpret_cast<const __half2*>(&v[i]);
+            const T2* h = reinterpret_cast<const T2*>(&v[i]);
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                const float2 f = __half22float2(h[t]);
+                const float2 f = to_float2(h[t]);
                 mx = fmaxf(mx, fmaxf(f.x, f.y));
             }
         }
@@ -197,10 +202,10 @@ __global__ void __launch_bounds__(SM_THREADS) softmax_rows_kernel(__half* __rest
     for (int i = 0; i < SM_MAXV; ++i) {
         const int j = threadIdx.x + i * SM_THREADS;
         if (j < nvec) {
-            const __half2* h = reinterpret_cast<const __half2*>(&v[i]);
+            const T2* h = reinterpret_cast<const T2*>(&v[i]);
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                const float2 f = __half22float2(h[t]);
+                const float2 f = to_float2(h[t]);
                 sum += exp2f(fmaf(f.x, scale_log2, -m)) + exp2f(fmaf(f.y, scale_log2, -m));
             }
         }
@@ -211,15 +216,14 @@ __global__ void __launch_bounds__(SM_THREADS) softmax_rows_kernel(__half* __rest
     for (int i = 0; i < SM_MAXV; ++i) {
         const int j = threadIdx.x + i * SM_THREADS;
         if (j < nvec) {
-            const __half2* h = reinterpret_cast<const __half2*>(&v[i]);
-            uint4 o;
-            __half2* ho = reinterpret_cast<__half2*>(&o);
+            const T2* h = reinterpret_cast<const T2*>(&v[i]);
+            uint32_t o[4];
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                const float2 f = __half22float2(h[t]);
-                ho[t] = __floats2half2_rn(exp2f(fmaf(f.x, scale_log2, -m)) * inv, exp2f(fmaf(f.y, scale_log2, -m)) * inv);
+                const float2 f = to_float2(h[t]);
+                o[t] = pack2<T>(exp2f(fmaf(f.x, scale_log2, -m)) * inv, exp2f(fmaf(f.y, scale_log2, -m)) * inv);
             }
-            row[j] = o;
+            row[j] = make_uint4(o[0], o[1], o[2], o[3]);
         }
     }
 }
@@ -228,15 +232,16 @@ __global__ void __launch_bounds__(SM_THREADS) softmax_rows_kernel(__half* __rest
 
 using namespace omg;
 
+template <typename T>
 static int softmax_rows_impl(void* x, long long rows, int cols, long long ld, float scale, void* stream_) {
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-    OMG_CHECK(x && rows >= 1 && rows <= 0x7fffffffLL, "omg_softmax_rows: bad arguments");
+    const char* fn = std::is_same<T, __half>::value ? "omg_softmax_rows" : "omg_softmax_rows_bf16";
+    OMG_CHECK(x && rows >= 1 && rows <= 0x7fffffffLL, "%s: bad arguments", fn);
     OMG_CHECK(cols >= 8 && cols % 8 == 0 && cols <= SM_THREADS * SM_MAXV * 8 && ld % 8 == 0 && ld >= cols,
-              "omg_softmax_rows: cols=%d must be a multiple of 8 and <= %d, ld a multiple of 8", cols,
-              SM_THREADS * SM_MAXV * 8);
-    OMG_CHECK(scale > 0.f, "omg_softmax_rows: scale must be positive");
-    OMG_CUDA(launch_pdl(softmax_rows_kernel, dim3((unsigned)rows), dim3(SM_THREADS), 0, stream,
-                        static_cast<__half*>(x), cols, ld, scale * 1.4426950408889634f));
+              "%s: cols=%d must be a multiple of 8 and <= %d, ld a multiple of 8", fn, cols, SM_THREADS * SM_MAXV * 8);
+    OMG_CHECK(scale > 0.f, "%s: scale must be positive", fn);
+    OMG_CUDA(launch_pdl(softmax_rows_kernel<T>, dim3((unsigned)rows), dim3(SM_THREADS), 0, stream,
+                        static_cast<T*>(x), cols, ld, scale * 1.4426950408889634f));
     return check_launch("softmax_rows_kernel");
 }
 
@@ -286,8 +291,14 @@ static int ctx_mix_impl(const void* ctx, const void* coef, void* out, int B, int
 
 // C-ABI entry points: launch, and - while this thread records a launch plan (omg_plan_record_begin) - remember the call
 extern "C" int omg_softmax_rows(void* x, long long rows, int cols, long long ld, float scale, void* stream_) {
-    const int rc = softmax_rows_impl(x, rows, cols, ld, scale, stream_);
-    if (rc == 0 && ::omg::plan_recording()) ::omg::plan_note([=](void* s) { return softmax_rows_impl(x, rows, cols, ld, scale, s); });
+    const int rc = softmax_rows_impl<__half>(x, rows, cols, ld, scale, stream_);
+    if (rc == 0 && ::omg::plan_recording()) ::omg::plan_note([=](void* s) { return softmax_rows_impl<__half>(x, rows, cols, ld, scale, s); });
+    return rc;
+}
+
+extern "C" int omg_softmax_rows_bf16(void* x, long long rows, int cols, long long ld, float scale, void* stream_) {
+    const int rc = softmax_rows_impl<__nv_bfloat16>(x, rows, cols, ld, scale, stream_);
+    if (rc == 0 && ::omg::plan_recording()) ::omg::plan_note([=](void* s) { return softmax_rows_impl<__nv_bfloat16>(x, rows, cols, ld, scale, s); });
     return rc;
 }
 

@@ -19,6 +19,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <type_traits>
 
 #include "../../include/omg_b200.h"
 #include "host_common.h"
@@ -46,10 +47,10 @@ struct alignas(64) GemmParams {
     int store_w, store_h;
     int img_w, img_h, img_b;
     int N, N_out;
-    const __half* bias;
-    const __half* rowvec;
+    const void* bias;          // element type of the kernel instantiation (fp16 | bf16)
+    const void* rowvec;
     int rowvec_ld;
-    const __half* residual;
+    const void* residual;
     int residual_ld;
     int act_silu;
     // LayerNorm folded into the GEMM pair (see omg_gemm_desc): statistics written by the producer's epilogue ...
@@ -114,9 +115,12 @@ __device__ __forceinline__ float gelu_exact(float x) { return 0.5f * x * (1.0f +
 //   1  + GroupNorm column statistics (convs, proj_out)
 //   2  + activations (SiLU, quick-GELU, erf / tanh GELU) and the fp32 residual-trunk twins (once-per-call MLPs, CLIP / SAM
 //      towers, OMG_TRUNK_F32)
-template <int BN, int EPI, int CTAS, int MT, int FEAT>
+// T is the 16-bit element type of every operand and of the output: __half, or __nv_bfloat16 (instantiated only with
+// FEAT 0 and OMG_EPI_NONE, what the VAE decoder uses).
+template <int BN, int EPI, int CTAS, int MT, int FEAT, typename T = __half>
 __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_constant__ GemmParams p) {
     constexpr bool kStats = FEAT >= 1, kExtra = FEAT >= 2;
+    using T2 = typename Pair<T>::type;
     static_assert(MT == 1 || CTAS == 1, "tall tiles are a single-CTA variant");
     static_assert(BN <= 256 || (CTAS == 2 && BN == 320 && EPI != OMG_EPI_GEGLU), "BN = 320 exists as a CTA-pair tile only");
     using Cfg = GemmCfg<BN, CTAS, MT>;
@@ -227,7 +231,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
     } else if (warp == 1) {
         // ------------------------------------------------------------- MMA issuer (one thread)
         if (lane == 0 && leader) {
-            constexpr uint32_t idesc = umma_idesc_f16(BM * CTAS, BN > 256 ? 160 : BN, false, false);
+            constexpr uint32_t idesc = umma_idesc_f16(BM * CTAS, BN > 256 ? 160 : BN, false, false,
+                                                      std::is_same<T, __nv_bfloat16>::value);
             int stage = 0;
             uint32_t phase = 0;
             int acc = 0;
@@ -323,8 +328,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
                         v = p.col_c2[cg + n];
                         c1 = p.col_c1[cg + n];
                     } else {
-                        if (p.bias) v += __half2float(p.bias[n]);
-                        if (p.rowvec && b < p.img_b) v += __half2float(p.rowvec[(size_t)b * p.rowvec_ld + n]);
+                        if (p.bias) v += to_float(static_cast<const T*>(p.bias)[n]);
+                        if (p.rowvec && b < p.img_b) v += to_float(static_cast<const T*>(p.rowvec)[(size_t)b * p.rowvec_ld + n]);
                     }
                 }
                 sbias[j] = v;
@@ -357,7 +362,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
             // ready), so their HBM/L2 latency hides behind the mainloop / the previous chunks
             uint4 res[2][4];
             const bool has_res = (EPI != OMG_EPI_GEGLU) && p.residual != nullptr && row_valid;
-            const __half* res_row = has_res ? p.residual + pix * (size_t)p.residual_ld + n0 : nullptr;
+            const T* res_row = has_res ? static_cast<const T*>(p.residual) + pix * (size_t)p.residual_ld + n0 : nullptr;
             auto load_res = [&](int c, uint4(&dst)[4]) {
                 if (has_res && c < NCH && n0 + c * 32 < p.N) {
                     const uint4* rp = reinterpret_cast<const uint4*>(res_row + c * 32);
@@ -404,10 +409,10 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
                     };
 #pragma unroll
                     for (int j = 0; j < 8; ++j)  // columns (4j, 4j+1) and (4j+2, 4j+3) are (value, gate) pairs
-                        outp[j] = pack_half2(pair_out(r0, 0, 4 * j), pair_out(r0, 0, 4 * j + 2));
+                        outp[j] = pack2<T>(pair_out(r0, 0, 4 * j), pair_out(r0, 0, 4 * j + 2));
 #pragma unroll
                     for (int j = 0; j < 8; ++j)
-                        outp[8 + j] = pack_half2(pair_out(r1, 32, 4 * j), pair_out(r1, 32, 4 * j + 2));
+                        outp[8 + j] = pack2<T>(pair_out(r1, 32, 4 * j), pair_out(r1, 32, 4 * j + 2));
                 } else {
                     uint32_t r[32];
                     tmem_ld_32x32(t_row + c * 32, r);
@@ -444,10 +449,10 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
 #pragma unroll
                         for (int j4 = 0; j4 < 4; ++j4) {
                             const uint4 u = resb[j4];
-                            const __half2* h2 = reinterpret_cast<const __half2*>(&u);
+                            const T2* h2 = reinterpret_cast<const T2*>(&u);
 #pragma unroll
                             for (int t = 0; t < 4; ++t) {
-                                const float2 f = __half22float2(h2[t]);
+                                const float2 f = to_float2(h2[t]);
                                 v[j4 * 8 + 2 * t] += f.x;
                                 v[j4 * 8 + 2 * t + 1] += f.y;
                             }
@@ -490,7 +495,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
                         }
                     }
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) outp[j] = pack_half2(v[2 * j], v[2 * j + 1]);
+                    for (int j = 0; j < 16; ++j) outp[j] = pack2<T>(v[2 * j], v[2 * j + 1]);
                 }
                 if constexpr (EPI != OMG_EPI_GEGLU && kStats) {
                     if (p.col_stats != nullptr && !row_valid) {  // rows outside the image count as zeros
@@ -524,9 +529,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
                             const int r = 2 * i + hp;
-                            const __half2 h2 = *reinterpret_cast<const __half2*>(
+                            const T2 h2 = *reinterpret_cast<const T2*>(
                                 sbuf + r * 64 + (((cp >> 2) ^ (i & 3)) << 4) + ((cp & 3) << 2));
-                            const float2 f = __half22float2(h2);
+                            const float2 f = to_float2(h2);
                             s0 += f.x;
                             q0 = fmaf(f.x, f.x, q0);
                             s1 += f.y;
@@ -589,20 +594,20 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const __grid_c
 
 // ------------------------------------------------------------------------------------------------ host
 static int view_to_tmap(CUtensorMap* m, const omg_view4& v, uint32_t box_c, uint32_t box_w, uint32_t box_h,
-                        CUtensorMapSwizzle sw) {
+                        CUtensorMapSwizzle sw, CUtensorMapDataType dt) {
     const uint64_t dims[4] = {(uint64_t)v.C, (uint64_t)v.W, (uint64_t)v.H, (uint64_t)v.B};
     const uint64_t strides[4] = {1, (uint64_t)v.sw, (uint64_t)v.sh, (uint64_t)v.sb};
     const uint32_t box[4] = {box_c, box_w, box_h, 1};
-    return make_tmap_f16(m, v.ptr, 4, dims, strides, box, sw);
+    return make_tmap_16b(m, v.ptr, 4, dims, strides, box, sw, dt);
 }
 
-template <int BN, int EPI, int CTAS, int MT, int FEAT>
+template <int BN, int EPI, int CTAS, int MT, int FEAT, typename T = __half>
 static int launch_gemm_f(const GemmParams& p, cudaStream_t stream) {
     using Cfg = GemmCfg<BN, CTAS, MT>;
     static bool configured = false;
     static int num_sms = 0;
     if (!configured) {
-        OMG_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, CTAS, MT, FEAT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        OMG_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BN, EPI, CTAS, MT, FEAT, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       Cfg::SMEM_BYTES));
         int dev = 0;
         OMG_CUDA(cudaGetDevice(&dev));
@@ -611,14 +616,19 @@ static int launch_gemm_f(const GemmParams& p, cudaStream_t stream) {
     }
     const int units = ((p.m_tiles + CTAS * MT - 1) / (CTAS * MT)) * p.n_tiles;
     const int grid = CTAS * std::min(units, num_sms / CTAS);
-    OMG_CUDA(launch_cluster(gemm_tc_kernel<BN, EPI, CTAS, MT, FEAT>, dim3(grid), dim3(GEMM_THREADS), Cfg::SMEM_BYTES, stream, CTAS, p));
+    OMG_CUDA(launch_cluster(gemm_tc_kernel<BN, EPI, CTAS, MT, FEAT, T>, dim3(grid), dim3(GEMM_THREADS), Cfg::SMEM_BYTES, stream, CTAS, p));
     return check_launch("gemm_tc_kernel");
 }
 
-// FEAT dispatch: 0 lean, 1 + GroupNorm column statistics, 2 + activations / fp32 twins (GEGLU launches are always lean)
-template <int BN, int EPI, int CTAS, int MT = 1>
+// FEAT dispatch: 0 lean, 1 + GroupNorm column statistics, 2 + activations / fp32 twins (GEGLU launches are always lean).
+// bf16 exists as the lean OMG_EPI_NONE variant only (gemm_impl rejects every other feature in bf16 mode): a larger
+// epilogue cost the hot fp16 instantiations 3..17 %, and the VAE decoder needs none of it.
+template <int BN, int EPI, int CTAS, int MT = 1, typename T = __half>
 static int launch_gemm(const GemmParams& p, cudaStream_t stream) {
-    if constexpr (EPI == OMG_EPI_GEGLU) {
+    if constexpr (std::is_same<T, __nv_bfloat16>::value) {
+        static_assert(EPI == OMG_EPI_NONE, "bf16 GEMMs have no activation epilogue");
+        return launch_gemm_f<BN, EPI, CTAS, MT, 0, T>(p, stream);
+    } else if constexpr (EPI == OMG_EPI_GEGLU) {
         return launch_gemm_f<BN, EPI, CTAS, MT, 0>(p, stream);
     } else {
         if (p.act_silu != 0 || p.residual_f32 != nullptr || p.out_f32 != nullptr) return launch_gemm_f<BN, EPI, CTAS, MT, 2>(p, stream);
@@ -677,6 +687,23 @@ static int pick_block_n(int N, int epilogue, long m_tiles, long k_plan, long k_b
     return best;
 }
 
+// the non-GEGLU tile shapes: CTA pairs (block_n 160 | 256 | 320), tall 256 x 160 tiles, single 128 x block_n tiles
+template <typename T>
+static int launch_tiles(const GemmParams& p, int bn, bool pair, bool tall, cudaStream_t stream) {
+    if (pair) {
+        if (bn == 320) return launch_gemm<320, OMG_EPI_NONE, 2, 1, T>(p, stream);
+        if (bn == 160) return launch_gemm<160, OMG_EPI_NONE, 2, 1, T>(p, stream);
+        return launch_gemm<256, OMG_EPI_NONE, 2, 1, T>(p, stream);
+    }
+    if (tall) return launch_gemm<160, OMG_EPI_NONE, 1, 2, T>(p, stream);
+    switch (bn) {
+        case 64: return launch_gemm<64, OMG_EPI_NONE, 1, 1, T>(p, stream);
+        case 128: return launch_gemm<128, OMG_EPI_NONE, 1, 1, T>(p, stream);
+        case 160: return launch_gemm<160, OMG_EPI_NONE, 1, 1, T>(p, stream);
+        default: return launch_gemm<256, OMG_EPI_NONE, 1, 1, T>(p, stream);
+    }
+}
+
 }  // namespace omg
 
 using namespace omg;
@@ -704,6 +731,18 @@ extern "C" int omg_gemm_colstats_blocks(int W, int H) {
 static int gemm_impl(const omg_gemm_desc* d, void* stream_) {
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
     OMG_CHECK(d != nullptr, "omg_gemm: null descriptor");
+    OMG_CHECK(d->dtype == OMG_DTYPE_F16 || d->dtype == OMG_DTYPE_BF16, "omg_gemm: unknown dtype %d", d->dtype);
+    const bool bf16 = d->dtype == OMG_DTYPE_BF16;
+    if (bf16) {  // exactly what the VAE decoder uses; see launch_gemm
+        OMG_CHECK(d->epilogue == OMG_EPI_NONE, "omg_gemm: bf16 supports no epilogue activation (GEGLU, SiLU, GELU): epilogue %d",
+                  d->epilogue);
+        OMG_CHECK(!d->row_stats_out && !d->row_stats_in, "omg_gemm: bf16 does not support the folded LayerNorm (row_stats_*)");
+        OMG_CHECK(!d->col_stats_out, "omg_gemm: bf16 does not support col_stats_out");
+        OMG_CHECK(!d->rowvec, "omg_gemm: bf16 does not support rowvec");
+        OMG_CHECK(d->w_group_planes == 0 && d->n_col_groups <= 1, "omg_gemm: bf16 does not support weight planes or column groups");
+        OMG_CHECK(!d->residual_f32 && !d->out_f32, "omg_gemm: bf16 does not support the fp32 twins (residual_f32 / out_f32)");
+    }
+    const CUtensorMapDataType dt = bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
     OMG_CHECK(d->n_a >= 1 && d->n_a <= OMG_MAX_A, "omg_gemm: n_a=%d out of range", d->n_a);
     OMG_CHECK(d->n_segs >= 1 && d->n_segs <= OMG_MAX_SEGS, "omg_gemm: n_segs=%d out of range", d->n_segs);
     OMG_CHECK(d->w && d->d.ptr, "omg_gemm: null weight/output pointer");
@@ -764,10 +803,10 @@ static int gemm_impl(const omg_gemm_desc* d, void* stream_) {
     OMG_CHECK(bn != 320 || (!geglu && d->N % 320 == 0), "omg_gemm: block_n=320 needs N %% 320 == 0 and no GEGLU");
     if (geglu) bn = 256;
     p.n_tiles = (d->N + bn - 1) / bn;
-    p.bias = static_cast<const __half*>(d->bias);
-    p.rowvec = static_cast<const __half*>(d->rowvec);
+    p.bias = d->bias;
+    p.rowvec = d->rowvec;
     p.rowvec_ld = d->rowvec_ld;
-    p.residual = static_cast<const __half*>(d->residual);
+    p.residual = d->residual;
     p.residual_ld = d->residual_ld;
     p.act_silu = act;  // 0 none, 1 SiLU, 2 quick_gelu, 3 erf-gelu, 4 tanh-gelu
     p.stats_out = static_cast<float*>(d->row_stats_out);
@@ -811,7 +850,7 @@ static int gemm_impl(const omg_gemm_desc* d, void* stream_) {
 
     for (int i = 0; i < d->n_a; ++i) {
         OMG_CHECK(d->a[i].ptr != nullptr, "omg_gemm: A view %d is null", i);
-        if (view_to_tmap(&p.a_maps[i], d->a[i], BK, tw, th, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (view_to_tmap(&p.a_maps[i], d->a[i], BK, tw, th, CU_TENSOR_MAP_SWIZZLE_128B, dt)) return 1;
     }
     for (int i = d->n_a; i < OMG_MAX_A; ++i) p.a_maps[i] = p.a_maps[0];
     {
@@ -819,7 +858,7 @@ static int gemm_impl(const omg_gemm_desc* d, void* stream_) {
         const uint64_t dims[2] = {(uint64_t)d->Ktot, (uint64_t)d->N * planes};
         const uint64_t strides[2] = {1, (uint64_t)d->Ktot};
         const uint32_t box[2] = {BK, (uint32_t)std::min(bn, 256)};
-        if (make_tmap_f16(&p.b_maps[0], d->w, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (make_tmap_16b(&p.b_maps[0], d->w, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, dt)) return 1;
         p.b_maps[1] = p.b_maps[0];
     }
     if (d->w2 != nullptr) {
@@ -827,9 +866,9 @@ static int gemm_impl(const omg_gemm_desc* d, void* stream_) {
         const uint64_t dims[2] = {(uint64_t)d->K2tot, (uint64_t)d->N};
         const uint64_t strides[2] = {1, (uint64_t)d->K2tot};
         const uint32_t box[2] = {BK, (uint32_t)std::min(bn, 256)};
-        if (make_tmap_f16(&p.b_maps[1], d->w2, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+        if (make_tmap_16b(&p.b_maps[1], d->w2, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, dt)) return 1;
     }
-    if (view_to_tmap(&p.d_map, d->d, 32, p.store_w, p.store_h, CU_TENSOR_MAP_SWIZZLE_64B)) return 1;
+    if (view_to_tmap(&p.d_map, d->d, 32, p.store_w, p.store_h, CU_TENSOR_MAP_SWIZZLE_64B, dt)) return 1;
 
     p.n_segs = d->n_segs;
     for (int s = 0; s < d->n_segs; ++s) {
@@ -867,26 +906,18 @@ static int gemm_impl(const omg_gemm_desc* d, void* stream_) {
             const uint64_t dims[2] = {(uint64_t)kt, (uint64_t)d->N * planes};
             const uint64_t strides[2] = {1, (uint64_t)kt};
             const uint32_t box[2] = {BK, (uint32_t)(bn == 320 ? 80 : bn / 2)};
-            if (make_tmap_f16(&p.b_maps[i], wp, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B)) return 1;
+            if (make_tmap_16b(&p.b_maps[i], wp, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, dt)) return 1;
         }
         if (!d->w2) p.b_maps[1] = p.b_maps[0];
         if (geglu) return launch_gemm<256, OMG_EPI_GEGLU, 2>(p, stream);
-        if (bn == 320) return launch_gemm<320, OMG_EPI_NONE, 2>(p, stream);
-        if (bn == 160) return launch_gemm<160, OMG_EPI_NONE, 2>(p, stream);
-        return launch_gemm<256, OMG_EPI_NONE, 2>(p, stream);
+        return bf16 ? launch_tiles<__nv_bfloat16>(p, bn, true, false, stream) : launch_tiles<__half>(p, bn, true, false, stream);
     }
     // tall tiles (256 x 160 per CTA): the narrow-N, long-enough-K GEMMs whose 128 x 160 tiles are L2-latency bound
     const bool tall = bn == 160 && !geglu && pair_ok &&
                       (d->cta_pair == 3 ||
                        (d->cta_pair == 0 && (prefer_tall || use_tall_tiles(p.m_tiles, p.n_tiles, k_blocks))));
-    if (tall) return launch_gemm<160, OMG_EPI_NONE, 1, 2>(p, stream);
     if (geglu) return launch_gemm<256, OMG_EPI_GEGLU, 1>(p, stream);
-    switch (bn) {
-        case 64: return launch_gemm<64, OMG_EPI_NONE, 1>(p, stream);
-        case 128: return launch_gemm<128, OMG_EPI_NONE, 1>(p, stream);
-        case 160: return launch_gemm<160, OMG_EPI_NONE, 1>(p, stream);
-        default: return launch_gemm<256, OMG_EPI_NONE, 1>(p, stream);
-    }
+    return bf16 ? launch_tiles<__nv_bfloat16>(p, bn, false, tall, stream) : launch_tiles<__half>(p, bn, false, tall, stream);
 }
 
 // C-ABI entry points: launch, and - while this thread records a launch plan (omg_plan_record_begin) - remember the call

@@ -36,8 +36,8 @@ PFN_encodeTiled get_encode_tiled() {
     return fn;
 }
 
-int make_tmap_f16(CUtensorMap* out, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_elems,
-                  const uint32_t* box, CUtensorMapSwizzle swizzle) {
+int make_tmap_16b(CUtensorMap* out, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_elems,
+                  const uint32_t* box, CUtensorMapSwizzle swizzle, CUtensorMapDataType dtype) {
     PFN_encodeTiled enc = get_encode_tiled();
     OMG_CHECK(enc != nullptr, "cuTensorMapEncodeTiled unavailable (no CUDA driver?)");
     cuuint64_t gdim[5], gstr[5];
@@ -54,7 +54,7 @@ int make_tmap_f16(CUtensorMap* out, const void* ptr, int rank, const uint64_t* d
         OMG_CHECK(box[i] >= 1 && box[i] <= 256, "tensor map box dim %d = %u out of range", i, box[i]);
     }
     OMG_CHECK((reinterpret_cast<uintptr_t>(ptr) & 15) == 0, "tensor map base pointer not 16 B aligned");
-    CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, rank, const_cast<void*>(ptr), gdim, gstr, bdim, estr,
+    CUresult r = enc(out, dtype, rank, const_cast<void*>(ptr), gdim, gstr, bdim, estr,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     OMG_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);

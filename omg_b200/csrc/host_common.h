@@ -92,9 +92,10 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
 // libcuda is resolved at run time through the runtime (the build box has no driver library to link against).
 PFN_encodeTiled get_encode_tiled();
 
-// fp16 tensor map of rank `rank` (<=5). dims[0] is the contiguous dimension. strides are in ELEMENTS for
-// dims[1..rank-1].  Out-of-bounds box elements read as zero / are clipped on store.
-int make_tmap_f16(CUtensorMap* out, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_elems,
-                  const uint32_t* box, CUtensorMapSwizzle swizzle);
+// Tensor map of 16-bit elements (`dtype` FLOAT16 or BFLOAT16) of rank `rank` (<=5). dims[0] is the contiguous dimension.
+// strides are in ELEMENTS for dims[1..rank-1].  Out-of-bounds box elements read as zero / are clipped on store.
+int make_tmap_16b(CUtensorMap* out, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_elems,
+                  const uint32_t* box, CUtensorMapSwizzle swizzle,
+                  CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_FLOAT16);
 
 }  // namespace omg

@@ -5,7 +5,13 @@
 // cat([hidden, skip], dim=1), diffusers UNet2DConditionModel up-blocks [3P]); the concatenation is never
 // materialised un-normalised: the apply pass writes the normalised, activated, concatenated tensor that the
 // following conv consumes through TMA.
+//
+// The normalising GroupNorm (omg_groupnorm) also exists for bf16 activations (omg_groupnorm_bf16, the VAE decoder with
+// weights that overflow fp16); the statistics are fp32 sums in both cases.
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
+
+#include <type_traits>
 
 #include "../../include/omg_b200.h"
 #include "host_common.h"
@@ -13,13 +19,15 @@
 
 namespace omg {
 
+template <typename T = __half>
 struct GnSrc {
-    const __half* x1;
-    const __half* x2;
+    const T* x1;
+    const T* x2;
     int C1, C2;  // channels of each source (C2 = 0 when unused); both multiples of 8
 };
 
-__device__ __forceinline__ uint4 gn_load8(const GnSrc& s, size_t pix, int c) {
+template <typename T>
+__device__ __forceinline__ uint4 gn_load8(const GnSrc<T>& s, size_t pix, int c) {
     // c is a multiple of 8 and an 8-vector never straddles the two sources
     if (c < s.C1) return *reinterpret_cast<const uint4*>(s.x1 + pix * s.C1 + c);
     return *reinterpret_cast<const uint4*>(s.x2 + pix * s.C2 + (c - s.C1));
@@ -29,7 +37,8 @@ __device__ __forceinline__ uint4 gn_load8(const GnSrc& s, size_t pix, int c) {
 //   pass 1  partial[b][split][g] = {sum, sumsq} over the CTA's rows    grid = (splits, B), block = (C/8, rows_par)
 //   pass 2  stats[b][g] = {mean, rstd}, partials summed in split order  grid = B, block = 32
 // Identical images in a batch therefore get bit-identical results (the reference's stage-1 rows are identical).
-__global__ void gn_partial_kernel(GnSrc s, int HW, int cpg, int rows_per_cta, float* __restrict__ partial) {
+template <typename T>
+__global__ void gn_partial_kernel(GnSrc<T> s, int HW, int cpg, int rows_per_cta, float* __restrict__ partial) {
     extern __shared__ float s_red[];  // [rows_par][C] sums, then [rows_par][C] squares
     griddep_launch_dependents();
     griddep_wait();
@@ -42,10 +51,10 @@ __global__ void gn_partial_kernel(GnSrc s, int HW, int cpg, int rows_per_cta, fl
 #pragma unroll
     for (int i = 0; i < 8; ++i) a[i] = q[i] = 0.f;
     auto acc8 = [&](const uint4& u) {
-        const __half2* h2 = reinterpret_cast<const __half2*>(&u);
+        const auto* h2 = reinterpret_cast<const typename Pair<T>::type*>(&u);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            const float2 f = __half22float2(h2[i]);
+            const float2 f = to_float2(h2[i]);
             a[2 * i] += f.x;
             q[2 * i] += f.x * f.x;
             a[2 * i + 1] += f.y;
@@ -100,19 +109,21 @@ __global__ void gn_partial_kernel(GnSrc s, int HW, int cpg, int rows_per_cta, fl
 }
 
 // per-(image, channel) affine of the normalisation: y = a * x + b with a = rstd * gamma, b = beta - mean * a
+template <typename T>
 __device__ __forceinline__ void gn_write_affine(float2* __restrict__ ab, int b, int C, int g, int cpg, int k0, int kstep,
-                                                float mean, float rstd, const __half* __restrict__ gamma,
-                                                const __half* __restrict__ beta) {
+                                                float mean, float rstd, const T* __restrict__ gamma,
+                                                const T* __restrict__ beta) {
     for (int k = k0; k < cpg; k += kstep) {
         const int c = g * cpg + k;
-        const float a = rstd * __half2float(gamma[c]);
-        ab[(size_t)b * C + c] = make_float2(a, __half2float(beta[c]) - mean * a);
+        const float a = rstd * to_float(gamma[c]);
+        ab[(size_t)b * C + c] = make_float2(a, to_float(beta[c]) - mean * a);
     }
 }
 
+template <typename T>
 __global__ void gn_finalize_kernel(const float* __restrict__ partial, int splits, float inv_n, float eps,
-                                   float2* __restrict__ ab, int C, int cpg, const __half* __restrict__ gamma,
-                                   const __half* __restrict__ beta) {
+                                   float2* __restrict__ ab, int C, int cpg, const T* __restrict__ gamma,
+                                   const T* __restrict__ beta) {
     const int b = blockIdx.x, g = threadIdx.x >> 5, lane = threadIdx.x & 31;  // block = 32 groups x 32 lanes
     griddep_launch_dependents();
     griddep_wait();
@@ -135,8 +146,9 @@ __global__ void gn_finalize_kernel(const float* __restrict__ partial, int splits
 // Apply pass: y = silu?(a[b, c] * x + b[b, c]).  block = (C/8 channel vectors, ry rows), grid = (row chunks, B): a thread
 // keeps ONE channel vector for all of its rows, so the affine is loaded once into registers and there is no index
 // arithmetic in the loop; four 16 B loads are in flight per thread, a warp's loads are contiguous runs of the row.
-__global__ void gn_apply_kernel(GnSrc s, int HW, int rows_per_cta, int silu, const float2* __restrict__ ab,
-                                __half* __restrict__ y) {
+template <typename T>
+__global__ void gn_apply_kernel(GnSrc<T> s, int HW, int rows_per_cta, int silu, const float2* __restrict__ ab,
+                                T* __restrict__ y) {
     griddep_launch_dependents();
     griddep_wait();
     const int C = s.C1 + s.C2;
@@ -158,11 +170,11 @@ __global__ void gn_apply_kernel(GnSrc s, int HW, int rows_per_cta, int silu, con
     const int r1 = min(r0 + rows_per_cta, HW);
     const int step = blockDim.y;
     auto emit = [&](const uint4& u, int r) {
-        const __half2* h2 = reinterpret_cast<const __half2*>(&u);
+        const auto* h2 = reinterpret_cast<const typename Pair<T>::type*>(&u);
         float v[8];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-            const float2 f = __half22float2(h2[i]);
+            const float2 f = to_float2(h2[i]);
             v[2 * i] = fmaf(a[2 * i], f.x, sft[2 * i]);
             v[2 * i + 1] = fmaf(a[2 * i + 1], f.y, sft[2 * i + 1]);
         }
@@ -170,10 +182,7 @@ __global__ void gn_apply_kernel(GnSrc s, int HW, int rows_per_cta, int silu, con
 #pragma unroll
             for (int i = 0; i < 8; ++i) v[i] = __fdividef(v[i], 1.0f + __expf(-v[i]));
         }
-        uint4 o;
-        __half2* oh = reinterpret_cast<__half2*>(&o);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) oh[i] = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
+        const uint4 o = make_uint4(pack2<T>(v[0], v[1]), pack2<T>(v[2], v[3]), pack2<T>(v[4], v[5]), pack2<T>(v[6], v[7]));
         *reinterpret_cast<uint4*>(y + ((size_t)b * HW + r) * C + c0) = o;
     };
     int r = r0 + threadIdx.y;
@@ -190,7 +199,8 @@ __global__ void gn_apply_kernel(GnSrc s, int HW, int rows_per_cta, int silu, con
     for (; r < r1; r += step) emit(gn_load8(s, (size_t)b * HW + r, c0), r);
 }
 
-static int launch_gn_apply(const GnSrc& s, int B, int HW, int silu, const float2* ab, __half* y, cudaStream_t stream) {
+template <typename T>
+static int launch_gn_apply(const GnSrc<T>& s, int B, int HW, int silu, const float2* ab, T* y, cudaStream_t stream) {
     const int C = s.C1 + s.C2;
     const int tx = C / 8;
     int ty = 512 / tx;
@@ -200,7 +210,7 @@ static int launch_gn_apply(const GnSrc& s, int B, int HW, int silu, const float2
     int rows_per_cta = (HW + 63) / 64;
     if (rows_per_cta < 4 * ty) rows_per_cta = 4 * ty;
     const int chunks = (HW + rows_per_cta - 1) / rows_per_cta;
-    OMG_CUDA(launch_pdl(gn_apply_kernel, dim3(chunks, B), dim3(tx, ty), 0, stream, s, HW, rows_per_cta, silu, ab, y));
+    OMG_CUDA(launch_pdl(gn_apply_kernel<T>, dim3(chunks, B), dim3(tx, ty), 0, stream, s, HW, rows_per_cta, silu, ab, y));
     return check_launch("gn_apply_kernel");
 }
 
@@ -373,16 +383,18 @@ __global__ void layernorm_kernel(const __half* __restrict__ x, const __half* __r
 
 using namespace omg;
 
+template <typename T>
 static int groupnorm_impl(const void* x1, int C1, const void* x2, int C2, int B, int HW, const void* gamma,
                              const void* beta, float eps, int silu, void* stats_ws, void* y, void* stream_) {
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
     const int C = C1 + C2;
-    OMG_CHECK(x1 && gamma && beta && stats_ws && y, "omg_groupnorm: null pointer");
-    OMG_CHECK(C1 > 0 && C1 % 8 == 0 && C2 >= 0 && C2 % 8 == 0 && (C2 == 0 || x2), "omg_groupnorm: bad channel split");
-    OMG_CHECK(C % 32 == 0 && C <= 2560, "omg_groupnorm: C=%d must be a multiple of 32 and <= 2560", C);
-    OMG_CHECK(B >= 1 && HW >= 1, "omg_groupnorm: empty input");
+    const char* fn = std::is_same<T, __half>::value ? "omg_groupnorm" : "omg_groupnorm_bf16";
+    OMG_CHECK(x1 && gamma && beta && stats_ws && y, "%s: null pointer", fn);
+    OMG_CHECK(C1 > 0 && C1 % 8 == 0 && C2 >= 0 && C2 % 8 == 0 && (C2 == 0 || x2), "%s: bad channel split", fn);
+    OMG_CHECK(C % 32 == 0 && C <= 2560, "%s: C=%d must be a multiple of 32 and <= 2560", fn, C);
+    OMG_CHECK(B >= 1 && HW >= 1, "%s: empty input", fn);
     const int cpg = C / 32;
-    GnSrc s{static_cast<const __half*>(x1), static_cast<const __half*>(x2), C1, C2};
+    GnSrc<T> s{static_cast<const T*>(x1), static_cast<const T*>(x2), C1, C2};
     const int tx = C / 8;
     int ty = 1024 / tx;
     if (ty > 16) ty = 16;
@@ -402,16 +414,16 @@ static int groupnorm_impl(const void* x1, int C1, const void* x2, int C2, int B,
     const size_t smem = (size_t)2 * ty * C * sizeof(float);
     static bool configured = false;
     if (!configured) {
-        OMG_CUDA(cudaFuncSetAttribute(gn_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 8192 * 4));  // ty * C <= 1024 * 8
+        OMG_CUDA(cudaFuncSetAttribute(gn_partial_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 8192 * 4));  // ty * C <= 1024 * 8
         configured = true;
     }
-    OMG_CUDA(launch_pdl(gn_partial_kernel, dim3(splits, B), dim3(tx, ty), smem, stream, s, HW, cpg, rows_per_cta, partial));
+    OMG_CUDA(launch_pdl(gn_partial_kernel<T>, dim3(splits, B), dim3(tx, ty), smem, stream, s, HW, cpg, rows_per_cta, partial));
     if (check_launch("gn_partial_kernel")) return 1;
-    OMG_CUDA(launch_pdl(gn_finalize_kernel, dim3(B), dim3(1024), 0, stream, (const float*)partial, splits,
-                        1.0f / ((float)HW * (float)cpg), eps, ab, C, cpg, static_cast<const __half*>(gamma),
-                        static_cast<const __half*>(beta)));
+    OMG_CUDA(launch_pdl(gn_finalize_kernel<T>, dim3(B), dim3(1024), 0, stream, (const float*)partial, splits,
+                        1.0f / ((float)HW * (float)cpg), eps, ab, C, cpg, static_cast<const T*>(gamma),
+                        static_cast<const T*>(beta)));
     if (check_launch("gn_finalize_kernel")) return 1;
-    return launch_gn_apply(s, B, HW, silu, ab, static_cast<__half*>(y), stream);
+    return launch_gn_apply(s, B, HW, silu, ab, static_cast<T*>(y), stream);
 }
 
 static int colstats_impl(const void* x, int C, int B, int HW, void* out, void* stream_) {
@@ -434,7 +446,7 @@ static int groupnorm_apply_impl(const void* x1, int C1, const void* part1, int r
     OMG_CHECK(C % 32 == 0 && C <= 2560, "omg_groupnorm_apply: C=%d must be a multiple of 32 and <= 2560", C);
     OMG_CHECK(B >= 1 && HW >= 1 && rb1 >= 1 && (C2 == 0 || rb2 >= 1), "omg_groupnorm_apply: empty input");
     const int cpg = C / 32;
-    GnSrc s{static_cast<const __half*>(x1), static_cast<const __half*>(x2), C1, C2};
+    GnSrc<> s{static_cast<const __half*>(x1), static_cast<const __half*>(x2), C1, C2};
     GnParts parts{static_cast<const float2*>(part1), static_cast<const float2*>(part2), C1, C2, rb1, rb2};
     float2* ab = static_cast<float2*>(stats_ws);  // [B][C] (a, b) of y = a x + b
     OMG_CUDA(launch_pdl(gn_reduce_kernel, dim3(32, B), dim3(256), 0, stream, parts, cpg, 1.0f / ((float)HW * (float)cpg), eps, ab,
@@ -468,8 +480,15 @@ static int layernorm_impl(const void* x, const void* gamma, const void* beta, vo
 // C-ABI entry points: launch, and - while this thread records a launch plan (omg_plan_record_begin) - remember the call
 extern "C" int omg_groupnorm(const void* x1, int C1, const void* x2, int C2, int B, int HW, const void* gamma,
                              const void* beta, float eps, int silu, void* stats_ws, void* y, void* stream_) {
-    const int rc = groupnorm_impl(x1, C1, x2, C2, B, HW, gamma, beta, eps, silu, stats_ws, y, stream_);
-    if (rc == 0 && ::omg::plan_recording()) ::omg::plan_note([=](void* s) { return groupnorm_impl(x1, C1, x2, C2, B, HW, gamma, beta, eps, silu, stats_ws, y, s); });
+    const int rc = groupnorm_impl<__half>(x1, C1, x2, C2, B, HW, gamma, beta, eps, silu, stats_ws, y, stream_);
+    if (rc == 0 && ::omg::plan_recording()) ::omg::plan_note([=](void* s) { return groupnorm_impl<__half>(x1, C1, x2, C2, B, HW, gamma, beta, eps, silu, stats_ws, y, s); });
+    return rc;
+}
+
+extern "C" int omg_groupnorm_bf16(const void* x1, int C1, const void* x2, int C2, int B, int HW, const void* gamma,
+                                  const void* beta, float eps, int silu, void* stats_ws, void* y, void* stream_) {
+    const int rc = groupnorm_impl<__nv_bfloat16>(x1, C1, x2, C2, B, HW, gamma, beta, eps, silu, stats_ws, y, stream_);
+    if (rc == 0 && ::omg::plan_recording()) ::omg::plan_note([=](void* s) { return groupnorm_impl<__nv_bfloat16>(x1, C1, x2, C2, B, HW, gamma, beta, eps, silu, stats_ws, y, s); });
     return rc;
 }
 

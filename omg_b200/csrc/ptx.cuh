@@ -3,6 +3,7 @@
 // kernels read as algorithms.  No CUTLASS/CuTe dependency.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -379,10 +380,10 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr, uint32_t
     return d;
 }
 
-// Instruction descriptor, kind::f16, fp16 A/B, fp32 D (cute::UMMA::InstrDescriptor bit layout).
-__host__ __device__ constexpr uint32_t umma_idesc_f16(int M, int N, bool a_mn_major, bool b_mn_major) {
+// Instruction descriptor, kind::f16, fp16 (or, with bf16 = true, bf16) A/B, fp32 D (cute::UMMA::InstrDescriptor bit layout).
+__host__ __device__ constexpr uint32_t umma_idesc_f16(int M, int N, bool a_mn_major, bool b_mn_major, bool bf16 = false) {
     return (1u << 4)                                   // D format f32
-           | (0u << 7) | (0u << 10)                    // A, B format f16
+           | ((bf16 ? 1u : 0u) << 7) | ((bf16 ? 1u : 0u) << 10)  // A, B format: 0 f16, 1 bf16
            | ((a_mn_major ? 1u : 0u) << 15) | ((b_mn_major ? 1u : 0u) << 16)
            | (static_cast<uint32_t>(N >> 3) << 17) | (static_cast<uint32_t>(M >> 4) << 24);
 }
@@ -395,5 +396,23 @@ __device__ __forceinline__ uint32_t pack_half2(float a, float b) {
     __half2 h = __floats2half2_rn(a, b);
     return *reinterpret_cast<uint32_t*>(&h);
 }
+
+__device__ __forceinline__ uint32_t pack_bf162(float a, float b) {
+    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<uint32_t*>(&h);
+}
+
+// The two 16-bit storage types of the activation paths: fp16 everywhere, bf16 for the VAE decoder with weights whose
+// activations exceed the fp16 range.  Both are 2 bytes wide, so TMA boxes, swizzles and vector widths do not change.
+template <typename T> struct Pair;
+template <> struct Pair<__half> { using type = __half2; };
+template <> struct Pair<__nv_bfloat16> { using type = __nv_bfloat162; };
+__device__ __forceinline__ float to_float(__half h) { return __half2float(h); }
+__device__ __forceinline__ float to_float(__nv_bfloat16 h) { return __bfloat162float(h); }
+__device__ __forceinline__ float2 to_float2(__half2 h) { return __half22float2(h); }
+__device__ __forceinline__ float2 to_float2(__nv_bfloat162 h) { return __bfloat1622float2(h); }
+template <typename T> __device__ __forceinline__ uint32_t pack2(float a, float b);
+template <> __device__ __forceinline__ uint32_t pack2<__half>(float a, float b) { return pack_half2(a, b); }
+template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float a, float b) { return pack_bf162(a, b); }
 
 }  // namespace omg

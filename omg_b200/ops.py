@@ -1,6 +1,8 @@
 """Host-side launchers: torch tensors (device memory + stream plumbing only) -> C-ABI descriptors.
 
-All activations are channels-last fp16: (B, H, W, C), equivalently (B, H*W tokens, C).
+All activations are channels-last fp16: (B, H, W, C), equivalently (B, H*W tokens, C).  `linear`, `conv3x3`,
+`upsample2x_conv3x3`, `groupnorm` and `softmax_rows` also run bf16 (the VAE decoder's path for weights whose activations
+overflow fp16): they take the element type from the input tensor and refuse operands of another type.
 """
 import ctypes as C
 
@@ -18,9 +20,23 @@ def _chk16(t: torch.Tensor):
         raise ValueError("expected a CUDA fp16 tensor (there is no CPU path)")
 
 
-def view4(t: torch.Tensor) -> L.View4:
-    """(B,H,W,C) tensor (any pixel strides, unit channel stride) or 2-D [M,K] matrix -> omg_view4."""
-    _chk16(t)
+_GEMM_DTYPES = {torch.float16: L.DTYPE_F16, torch.bfloat16: L.DTYPE_BF16}
+
+
+def _same_dtype(x: torch.Tensor, *others) -> torch.dtype:
+    """x.dtype, after checking that x is a CUDA fp16 | bf16 tensor and that every other operand given has its type."""
+    if not x.is_cuda or x.dtype not in _GEMM_DTYPES:
+        raise ValueError("expected a CUDA fp16 or bf16 tensor (there is no CPU path)")
+    for t in others:
+        if t is not None and t.dtype != x.dtype:
+            raise ValueError(f"mixed operand dtypes: input is {x.dtype}, an operand is {t.dtype}")
+    return x.dtype
+
+
+def view4(t: torch.Tensor, dtype: torch.dtype = torch.float16) -> L.View4:
+    """(B,H,W,C) tensor (any pixel strides, unit channel stride) or 2-D [M,K] matrix of `dtype` -> omg_view4."""
+    if _same_dtype(t) != dtype:
+        raise ValueError(f"expected a CUDA {dtype} tensor, got {t.dtype}")
     if t.dim() == 2:
         assert t.stride(1) == 1
         return L.View4(t.data_ptr(), t.shape[1], t.shape[0], 1, 1, t.stride(0), t.stride(0) * t.shape[0],
@@ -71,8 +87,9 @@ class LaunchPlan:
 
 def gemm(a_views, segs, w, N, Ktot, d_view, bias=None, rowvec=None, rowvec_ld=0, residual=None, residual_ld=0,
          epilogue=L.EPI_NONE, block_n=0, w2=None, stats_out=None, ln=None, cta_pair=0, row_groups=None, colstats=None,
-         residual_f32=None, out_f32=None):
+         residual_f32=None, out_f32=None, dtype=torch.float16):
     d = L.GemmDesc()
+    d.dtype = _GEMM_DTYPES[dtype]
     if residual_f32 is not None:   # [pixels, N] fp32 twins of the residual trunk (see omg_gemm_desc)
         d.residual_f32, d.residual_f32_ld = residual_f32.data_ptr(), residual_f32.stride(-2)
     if out_f32 is not None:
@@ -135,31 +152,31 @@ def linear(x, w, bias=None, residual=None, out=None, epilogue=L.EPI_NONE, extra=
     `extra` = list of (tensor [M,Ki], column offset into w): further K-segments of the same weight matrix.
     `lora`  = (t [M,R], w2 [N,R]): un-merged LoRA delta  t @ w2^T  with t = A x (scales folded into w2).
     """
-    _chk16(x)
+    dt = _same_dtype(x, w, bias, residual, out, *[t for t, _ in (extra or [])], *(lora or ()))
     M, K = x.shape
     N, Ktot = w.shape
     if row_groups is not None:
         N //= len(row_groups)
     n_out = N // 2 if epilogue == L.EPI_GEGLU else N
     if out is None:
-        out = torch.empty((M, n_out), dtype=torch.float16, device=x.device)
-    views = [view4(x)]
+        out = torch.empty((M, n_out), dtype=dt, device=x.device)
+    views = [view4(x, dt)]
     segs = [(0, 0, 0, 0, K, 0)]
     for t, off in (extra or []):
-        views.append(view4(t))
+        views.append(view4(t, dt))
         segs.append((len(views) - 1, 0, 0, 0, t.shape[1], off))
     w2 = None
     if lora is not None:
         t, w2 = lora
-        views.append(view4(t))
+        views.append(view4(t, dt))
         segs.append((len(views) - 1, 0, 0, 0, t.shape[1], 0, 1))
     # colstats: partials [B, rb, N, 2] of an output of B images x HW tokens; the [M, N] GEMM sees them as one image
     # of M rows, which is the same memory when no 128-row tile straddles two images (HW % 128 == 0, caller's duty)
     cs = None if colstats is None else (colstats.view(1, -1, colstats.shape[2], 2), 0)
-    gemm(views, segs, w, N, Ktot, view4(out), bias=bias, residual=residual,
+    gemm(views, segs, w, N, Ktot, view4(out, dt), bias=bias, residual=residual,
          residual_ld=0 if residual is None else residual.stride(0), epilogue=epilogue, block_n=block_n, w2=w2,
          stats_out=stats_out, ln=ln, cta_pair=cta_pair, row_groups=row_groups, colstats=cs,
-         residual_f32=residual_f32, out_f32=out_f32)
+         residual_f32=residual_f32, out_f32=out_f32, dtype=dt)
     return out
 
 
@@ -174,19 +191,20 @@ def conv3x3(x, w, bias=None, rowvec=None, residual=None, out=None, shortcut=None
     shortcut = list of (tensor (B,H,W,Ci), weight column offset): 1x1-conv K-segments added to the same accumulator
     (ResnetBlock2D conv_shortcut).  rowvec [B, N] is added per image (time-embedding projection).
     """
+    dt = _same_dtype(x, w, bias, rowvec, residual, out, *[t for t, _ in (shortcut or [])])
     B, H, W, Cin = x.shape
     N, Ktot = w.shape
     if out is None:
-        out = torch.empty((B, H, W, N), dtype=torch.float16, device=x.device)
-    views = [view4(x)]
+        out = torch.empty((B, H, W, N), dtype=dt, device=x.device)
+    views = [view4(x, dt)]
     segs = _taps3x3(Cin)
     for t, off in (shortcut or []):
-        views.append(view4(t))
+        views.append(view4(t, dt))
         segs.append((len(views) - 1, 0, 0, 0, t.shape[3], off))
-    gemm(views, segs, w, N, Ktot, view4(out), bias=bias, rowvec=rowvec,
+    gemm(views, segs, w, N, Ktot, view4(out, dt), bias=bias, rowvec=rowvec,
          rowvec_ld=0 if rowvec is None else rowvec.stride(0),
          residual=residual, residual_ld=0 if residual is None else N, block_n=block_n, cta_pair=cta_pair,
-         colstats=None if colstats is None else (colstats, 0), residual_f32=residual_f32, out_f32=out_f32)
+         colstats=None if colstats is None else (colstats, 0), residual_f32=residual_f32, out_f32=out_f32, dtype=dt)
     return out
 
 
@@ -209,20 +227,22 @@ def conv3x3_s2(x, w, bias=None, out=None, block_n=0, colstats=None):
     return out
 
 
-def upsample2x_conv3x3(x, w, bias=None, out=None, block_n=0, colstats=None):
+def upsample2x_conv3x3(x, w, bias=None, out=None, block_n=0, colstats=None, cta_pair=0):
     """nearest-2x upsample followed by 3x3 conv (Upsample2D) without materialising the upsampled tensor:
     each output phase (py,px) is a 9-tap conv over x with shifted taps, stored through a strided output view."""
+    dt = _same_dtype(x, w, bias, out)
     B, H, W, Cin = x.shape
     N, Ktot = w.shape
     if out is None:
-        out = torch.empty((B, 2 * H, 2 * W, N), dtype=torch.float16, device=x.device)
-    xv = view4(x)
+        out = torch.empty((B, 2 * H, 2 * W, N), dtype=dt, device=x.device)
+    xv = view4(x, dt)
     off = {0: (-1, 0, 0), 1: (0, 0, 1)}
     for py in range(2):
         for px in range(2):
             segs = [(0, off[px][kx], off[py][ky], 0, Cin, (ky * 3 + kx) * Cin) for ky in range(3) for kx in range(3)]
             cs = None if colstats is None else (colstats, (py * 2 + px) * colstats_blocks(W, H))
-            gemm([xv], segs, w, N, Ktot, view4(out[:, py::2, px::2, :]), bias=bias, block_n=block_n, colstats=cs)
+            gemm([xv], segs, w, N, Ktot, view4(out[:, py::2, px::2, :], dt), bias=bias, block_n=block_n, colstats=cs, dtype=dt,
+                 cta_pair=cta_pair)
     return out
 
 
@@ -247,20 +267,21 @@ def attention(q, k, v, out, heads, n_q, n_kv, items, q_col0=0, k_col0=0, v_col0=
 
 
 def groupnorm(x1, gamma, beta, eps, silu, x2=None, out=None, stats_ws=None):
-    """GroupNorm(32)(cat([x1, x2], channel)) [+ SiLU]; x: (B, H, W, C) or (B, HW, C)."""
-    _chk16(x1)
+    """GroupNorm(32)(cat([x1, x2], channel)) [+ SiLU]; x: (B, H, W, C) or (B, HW, C), fp16 or bf16 (gamma, beta, x2 and
+    out of the same type)."""
+    dt = _same_dtype(x1, gamma, beta, x2, out)
     B = x1.shape[0]
     C1 = x1.shape[-1]
     HW = x1.numel() // (B * C1)
     C2 = 0 if x2 is None else x2.shape[-1]
     assert x1.is_contiguous() and (x2 is None or x2.is_contiguous())
     if out is None:
-        out = torch.empty((*x1.shape[:-1], C1 + C2), dtype=torch.float16, device=x1.device)
+        out = torch.empty((*x1.shape[:-1], C1 + C2), dtype=dt, device=x1.device)
     if stats_ws is None:
         stats_ws = torch.empty(B * (10240 + 64 * 256), dtype=torch.float32, device=x1.device)
-    L.check(L.load().omg_groupnorm(x1.data_ptr(), C1, _ptr(x2), C2, B, HW, gamma.data_ptr(), beta.data_ptr(),
-                                   float(eps), int(silu), stats_ws.data_ptr(), out.data_ptr(), _stream()),
-            "omg_groupnorm")
+    name = "omg_groupnorm" if dt == torch.float16 else "omg_groupnorm_bf16"
+    L.check(getattr(L.load(), name)(x1.data_ptr(), C1, _ptr(x2), C2, B, HW, gamma.data_ptr(), beta.data_ptr(),
+                                    float(eps), int(silu), stats_ws.data_ptr(), out.data_ptr(), _stream()), name)
     return out
 
 
@@ -385,11 +406,11 @@ def axpy(a, b, alpha=1.0, out=None):
 
 
 def softmax_rows(x, scale=1.0):
-    """In-place softmax(scale * x) over the last dimension of a 2-D fp16 matrix (rows may be strided)."""
-    _chk16(x)
+    """In-place softmax(scale * x) over the last dimension of a 2-D fp16 | bf16 matrix (rows may be strided)."""
+    dt = _same_dtype(x)
     assert x.dim() == 2 and x.stride(1) == 1
-    L.check(L.load().omg_softmax_rows(_ptr(x), x.shape[0], x.shape[1], x.stride(0), float(scale), _stream()),
-            "omg_softmax_rows")
+    name = "omg_softmax_rows" if dt == torch.float16 else "omg_softmax_rows_bf16"
+    L.check(getattr(L.load(), name)(_ptr(x), x.shape[0], x.shape[1], x.stride(0), float(scale), _stream()), name)
     return x
 
 

@@ -9,12 +9,17 @@ runs as scores = omg_gemm(Q, K), `omg_softmax_rows`, out = omg_gemm(P, V^T): 512
 550 GFLOP GEMMs.  `post_quant_conv` (1x1, 4 -> 4) carries the 1 / scaling_factor and is padded to the 8-channel
 granularity of the TMA path.
 
-Precision: fp16 storage / fp32 accumulation like the UNet.  The reference up-casts this module to fp32 because the
-original SDXL VAE weights overflow fp16 activations; with such weights use the fp16-safe re-export of the VAE
-(same architecture and keys) - a bf16 activation path is not built.
+Precision: fp16 or bf16 storage, fp32 accumulation.  The reference up-casts this module to fp32 because the original
+SDXL VAE weights overflow fp16 activations (the VAE config's `force_upcast`, lora_pipeline.py:635-646).  bf16 has
+fp32's exponent range, so `PackedVaeDecoder(..., dtype=torch.bfloat16)` decodes those weights with the same kernels
+(bf16 operands on the same tensor-core path; fp32 GroupNorm statistics); fp16 (the default) suits the fp16-safe
+re-export of the weights and is a little more accurate.  `PackedVaeDecoder.from_pretrained` picks the type from
+`force_upcast`, the signal the reference uses for its fp32 up-cast.
 """
+import json
+import os
 from dataclasses import dataclass
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import torch
 
@@ -38,8 +43,25 @@ class VaeConfig:
         return VaeConfig(block_out_channels=(64, 64, 128, 128))
 
 
-def _f16(t, dev):
-    return t.to(device=dev, dtype=torch.float16).contiguous()
+def vae_config_from(sd: Dict[str, torch.Tensor], config: Optional[dict] = None) -> Tuple[VaeConfig, torch.dtype]:
+    """(VaeConfig, activation dtype) of a diffusers AutoencoderKL: from its `config.json` dict when given (widths,
+    `scaling_factor`; `force_upcast`, diffusers' default true, selects bf16 and false fp16), else inferred from the
+    decoder's parameter shapes, with `VaeConfig`'s scaling factor and bf16 (the type that holds any SDXL VAE)."""
+    if config is not None:
+        d = VaeConfig()
+        cfg = VaeConfig(block_out_channels=tuple(config.get("block_out_channels", d.block_out_channels)),
+                        layers_per_block=int(config.get("layers_per_block", d.layers_per_block)),
+                        latent_channels=int(config.get("latent_channels", d.latent_channels)),
+                        out_channels=int(config.get("out_channels", d.out_channels)),
+                        scaling_factor=float(config.get("scaling_factor", d.scaling_factor)))
+        return cfg, (torch.bfloat16 if config.get("force_upcast", True) else torch.float16)
+    n_up = 1 + max(int(k.split(".")[2]) for k in sd if k.startswith("decoder.up_blocks."))
+    # up block i runs at width block_out_channels[n_up - 1 - i]
+    rev = [sd[f"decoder.up_blocks.{i}.resnets.0.conv1.weight"].shape[0] for i in range(n_up)]
+    n_res = 1 + max(int(k.split(".")[4]) for k in sd if k.startswith("decoder.up_blocks.0.resnets."))
+    cfg = VaeConfig(block_out_channels=tuple(reversed(rev)), layers_per_block=n_res - 1,
+                    latent_channels=sd["post_quant_conv.weight"].shape[0], out_channels=sd["decoder.conv_out.weight"].shape[0])
+    return cfg, torch.bfloat16
 
 
 def vae_decoder_param_shapes(cfg: VaeConfig) -> Dict[str, Tuple[int, ...]]:
@@ -101,15 +123,22 @@ def vae_decoder_flops(cfg: VaeConfig, h: int, w: int) -> float:
 
 
 class PackedVaeDecoder:
-    """Weights of `post_quant_conv` + `decoder.*` (diffusers AutoencoderKL key layout) repacked once for the kernels."""
+    """Weights of `post_quant_conv` + `decoder.*` (diffusers AutoencoderKL key layout) repacked once for the kernels.
+    `dtype` (fp16 | bf16) is the type the weights are packed in and the activations are decoded in."""
 
-    def __init__(self, state_dict: Dict[str, torch.Tensor], cfg: VaeConfig = VaeConfig(), device="cuda"):
-        self.cfg, self.device = cfg, torch.device(device)
+    def __init__(self, state_dict: Dict[str, torch.Tensor], cfg: VaeConfig = VaeConfig(), device="cuda",
+                 dtype: torch.dtype = torch.float16):
+        self.cfg, self.device, self.dtype = cfg, torch.device(device), dtype
         if self.device.type != "cuda":
             raise RuntimeError("the B200 path needs a CUDA device (there is no CPU fallback)")
+        if dtype not in (torch.float16, torch.bfloat16):
+            raise ValueError(f"the VAE decoder runs fp16 or bf16, not {dtype}")
         sd = {k: v.float() for k, v in state_dict.items() if k.startswith(("decoder.", "post_quant_conv."))}
         dev, p = self.device, {}
         self.p = p
+
+        def _cast(t, dev):  # packed in the decode type (fp16 | bf16)
+            return t.to(device=dev, dtype=dtype).contiguous()
 
         def conv(name, pad_in=0, pad_out=0):
             w, b = sd[name + ".weight"], sd[name + ".bias"]
@@ -122,15 +151,15 @@ class PackedVaeDecoder:
 
         def res(name):
             for i in ("1", "2"):
-                p[f"{name}.g{i}"] = _f16(sd[f"{name}.norm{i}.weight"], dev)
-                p[f"{name}.b{i}"] = _f16(sd[f"{name}.norm{i}.bias"], dev)
+                p[f"{name}.g{i}"] = _cast(sd[f"{name}.norm{i}.weight"], dev)
+                p[f"{name}.b{i}"] = _cast(sd[f"{name}.norm{i}.bias"], dev)
             w1, b1 = conv(name + ".conv1")
             w2, b2 = conv(name + ".conv2")
             if name + ".conv_shortcut.weight" in sd:  # 1x1 shortcut: extra K columns of conv2, biases summed
                 w2 = torch.cat([w2, sd[name + ".conv_shortcut.weight"].flatten(1)], dim=1)
                 b2 = b2 + sd[name + ".conv_shortcut.bias"]
-            p[name + ".w1"], p[name + ".bias1"] = _f16(w1, dev), _f16(b1, dev)
-            p[name + ".w2"], p[name + ".bias2"] = _f16(w2, dev), _f16(b2, dev)
+            p[name + ".w1"], p[name + ".bias1"] = _cast(w1, dev), _cast(b1, dev)
+            p[name + ".w2"], p[name + ".bias2"] = _cast(w2, dev), _cast(b2, dev)
 
         lc = cfg.latent_channels
         pad = (-lc) % 8
@@ -139,17 +168,17 @@ class PackedVaeDecoder:
         wpq[:lc, :lc] = sd["post_quant_conv.weight"].flatten(1) / cfg.scaling_factor
         bpq = torch.zeros(lc + pad)
         bpq[:lc] = sd["post_quant_conv.bias"]
-        p["pq.w"], p["pq.b"] = _f16(wpq, dev), _f16(bpq, dev)
+        p["pq.w"], p["pq.b"] = _cast(wpq, dev), _cast(bpq, dev)
         w, b = conv("decoder.conv_in", pad_in=pad)
-        p["conv_in.w"], p["conv_in.b"] = _f16(w, dev), _f16(b, dev)
+        p["conv_in.w"], p["conv_in.b"] = _cast(w, dev), _cast(b, dev)
         top = cfg.block_out_channels[-1]
         res("decoder.mid_block.resnets.0")
         a = "decoder.mid_block.attentions.0"
-        p["attn.g"], p["attn.b"] = _f16(sd[a + ".group_norm.weight"], dev), _f16(sd[a + ".group_norm.bias"], dev)
+        p["attn.g"], p["attn.b"] = _cast(sd[a + ".group_norm.weight"], dev), _cast(sd[a + ".group_norm.bias"], dev)
         s = top ** -0.5  # softmax scale folded into the query projection
-        p["attn.wqkv"] = _f16(torch.cat([sd[a + ".to_q.weight"] * s, sd[a + ".to_k.weight"], sd[a + ".to_v.weight"]]), dev)
-        p["attn.bqkv"] = _f16(torch.cat([sd[a + ".to_q.bias"] * s, sd[a + ".to_k.bias"], sd[a + ".to_v.bias"]]), dev)
-        p["attn.wo"], p["attn.bo"] = _f16(sd[a + ".to_out.0.weight"], dev), _f16(sd[a + ".to_out.0.bias"], dev)
+        p["attn.wqkv"] = _cast(torch.cat([sd[a + ".to_q.weight"] * s, sd[a + ".to_k.weight"], sd[a + ".to_v.weight"]]), dev)
+        p["attn.bqkv"] = _cast(torch.cat([sd[a + ".to_q.bias"] * s, sd[a + ".to_k.bias"], sd[a + ".to_v.bias"]]), dev)
+        p["attn.wo"], p["attn.bo"] = _cast(sd[a + ".to_out.0.weight"], dev), _cast(sd[a + ".to_out.0.bias"], dev)
         res("decoder.mid_block.resnets.1")
         self.n_up = len(cfg.block_out_channels)
         for i in range(self.n_up):
@@ -157,11 +186,26 @@ class PackedVaeDecoder:
                 res(f"decoder.up_blocks.{i}.resnets.{j}")
             if i < self.n_up - 1:
                 w, b = conv(f"decoder.up_blocks.{i}.upsamplers.0.conv")
-                p[f"up{i}.w"], p[f"up{i}.b"] = _f16(w, dev), _f16(b, dev)
-        p["out.g"], p["out.b"] = _f16(sd["decoder.conv_norm_out.weight"], dev), _f16(sd["decoder.conv_norm_out.bias"], dev)
+                p[f"up{i}.w"], p[f"up{i}.b"] = _cast(w, dev), _cast(b, dev)
+        p["out.g"], p["out.b"] = _cast(sd["decoder.conv_norm_out.weight"], dev), _cast(sd["decoder.conv_norm_out.bias"], dev)
         w, b = conv("decoder.conv_out", pad_out=(-cfg.out_channels) % 8)
-        p["conv_out.w"], p["conv_out.b"] = _f16(w, dev), _f16(b, dev)
+        p["conv_out.w"], p["conv_out.b"] = _cast(w, dev), _cast(b, dev)
         self._ws = None
+
+    @classmethod
+    def from_pretrained(cls, path: str, device="cuda") -> "PackedVaeDecoder":
+        """A diffusers VAE directory (`config.json` + `diffusion_pytorch_model[.fp16].safetensors`), or a checkpoint root
+        with a `vae/` subfolder.  The decode type follows the config's `force_upcast` (see `vae_config_from`)."""
+        from .checkpoints import load_unet_weights
+        sub = "vae" if os.path.isdir(os.path.join(path, "vae")) else ""
+        sd = load_unet_weights(path, subfolder=sub)
+        cfg_path = os.path.join(path, sub, "config.json")
+        config = None
+        if os.path.isfile(cfg_path):
+            with open(cfg_path) as f:
+                config = json.load(f)
+        cfg, dtype = vae_config_from(sd, config)
+        return cls(sd, cfg, device=device, dtype=dtype)
 
     # ------------------------------------------------------------------------------------------------ blocks
     def _stats_ws(self, B):
@@ -188,8 +232,8 @@ class PackedVaeDecoder:
         N = H * W
         n = ops.groupnorm(x, p["attn.g"], p["attn.b"], 1e-6, 0, stats_ws=self._stats_ws(B))
         qkv = ops.linear(n.view(B * N, C), p["attn.wqkv"], bias=p["attn.bqkv"]).view(B, N, 3 * C)
-        o = torch.empty((B, N, C), dtype=torch.float16, device=x.device)
-        scores = torch.empty((N, N), dtype=torch.float16, device=x.device)
+        o = torch.empty((B, N, C), dtype=x.dtype, device=x.device)
+        scores = torch.empty((N, N), dtype=x.dtype, device=x.device)
         for b in range(B):  # one image at a time: the score matrix is N x N (512 MB at 128 x 128 latents)
             q, k, v = qkv[b, :, :C], qkv[b, :, C:2 * C], qkv[b, :, 2 * C:]
             ops.linear(q.contiguous(), k.contiguous(), out=scores)   # (Q / sqrt(C)) K^T
@@ -202,11 +246,12 @@ class PackedVaeDecoder:
     # ------------------------------------------------------------------------------------------------ decode
     @torch.no_grad()
     def decode(self, latents: torch.Tensor) -> torch.Tensor:
-        """(B, 4, h, w) latents (as the pipelines return them) -> (B, 3, 8h, 8w) fp16 image, nominally in [-1, 1]."""
+        """(B, 4, h, w) latents (as the pipelines return them) -> (B, 3, 8h, 8w) image in the decode type, nominally in
+        [-1, 1]."""
         cfg, p = self.cfg, self.p
         B, lc, h, w = latents.shape
         pad = (-lc) % 8
-        z = torch.zeros((B, h, w, lc + pad), dtype=torch.float16, device=self.device)
+        z = torch.zeros((B, h, w, lc + pad), dtype=self.dtype, device=self.device)
         z[..., :lc] = latents.to(self.device).permute(0, 2, 3, 1)
         z = ops.linear(z.view(B * h * w, lc + pad), p["pq.w"], bias=p["pq.b"]).view(B, h, w, lc + pad)
         x = ops.conv3x3(z, p["conv_in.w"], bias=p["conv_in.b"])
@@ -229,8 +274,12 @@ class PackedVaeDecoder:
         if not bool(torch.isfinite(dec).all()):
             # fp16 activations overflow with the original SDXL VAE weights (the reference up-casts this module to
             # fp32 for that reason, lora_pipeline.py:635-646): refuse to hand back NaN / black images
-            raise FloatingPointError("VAE decode produced non-finite values in fp16: use the fp16-safe SDXL VAE "
-                                     "weights (same keys) or output_type='latent'")
+            if self.dtype == torch.float16:
+                raise FloatingPointError("VAE decode produced non-finite values in fp16: decode in bf16 "
+                                         "(PackedVaeDecoder(..., dtype=torch.bfloat16), or from_pretrained on a VAE whose "
+                                         "config has force_upcast), use the fp16-safe SDXL VAE weights (same keys), or "
+                                         "output_type='latent'")
+            raise FloatingPointError("VAE decode produced non-finite values in bf16")
         img = (dec / 2 + 0.5).clamp(0, 1)
         if output_type == "pt":
             return img
